@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (oracle port)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + what the last timed step computed, as .npy
 
 Workload (config.workload): BASELINE.json configs[2] -- 1 006 065 Gaussians (the test_garden crop tiled
 3x3, SURVEY.md section 8(d)), one 1920x1080 view per GPU, SH degree 3, dense (packed=False).
@@ -112,6 +113,26 @@ def measured_peak_gbs() -> tuple[float, str]:
         except Exception:
             pass
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_ROWS = 65536  # Gaussians whose gradients --dump-outputs writes (the full SH gradient alone is 193 MB)
+
+
+def dump_outputs(out_dir: str, render_colors, render_alphas, loss, grads: dict) -> None:
+    """Writes what the timed step returns to its caller as float32 DIR/<name>.npy: render_colors, render_alphas, loss
+    and v_<param>, the gradients of a fixed seeded sample of DUMP_ROWS Gaussians (their indices in gaussian_rows.npy,
+    float64); about 50 MB at the default workload.  The inputs are seeded, so two builds can be compared file by file."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = grads["means"].shape[0]
+    rows = np.sort(np.random.RandomState(0).choice(n, min(DUMP_ROWS, n), replace=False))
+    idx = torch.from_numpy(rows).to(grads["means"].device)
+    arrays = {"render_colors": render_colors, "render_alphas": render_alphas, "loss": loss.reshape(1)}
+    arrays.update({"v_" + k: g[idx] for k, g in grads.items()})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "gaussian_rows.npy"), rows.astype(np.float64))
 
 
 def build_scene():
@@ -409,7 +430,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-trainer", action="store_true", help="skip the cfg5 trainer-loop runs (about 2 minutes)")
     ap.add_argument("--trainer-steps", type=int, default=700)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -497,6 +521,8 @@ def main():
             dev_in[slot][2].copy_(target_host_u8 if e2e_u8 else target_host, non_blocking=True)
             copy_done[slot].record(copy_stream)
 
+    last_out = {}  # outputs of the latest step, kept only for --dump-outputs
+
     def step(e2e: bool, slot: int = 0):
         if e2e:
             torch.cuda.current_stream().wait_event(copy_done[slot])
@@ -515,6 +541,8 @@ def main():
         loss.backward()
         if world > 1:
             all_reduce_grads()  # the 59 floats / Gaussian (SURVEY.md section 8e), one launch, in place
+        if args.dump_outputs:
+            last_out.update(render_colors=rc, render_alphas=ra, loss=loss)
         if e2e:
             consumed[slot].record()
             loss_host.copy_(loss.detach(), non_blocking=True)
@@ -571,6 +599,8 @@ def main():
     ms_dev = timed(False, args.steps)
     ms_e2e = timed(True, args.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **last_out, grads={k: params[k].grad for k in grad_names})
 
     # ---- N > 1 diagnostics (outside the timed regions): where a DP step spends its time on every rank, and the
     # same job (world views / step over the same Gaussians, every gradient summed over all views) laid out the
@@ -760,7 +790,7 @@ def main():
             ref_cuda = run_ref_cuda(params, vm_dev, K_dev, target_dev, args.steps)
             ref_stock = run_ref_cuda_stock(params, vm_dev, K_dev, target_dev, args.steps)
             try:
-                big_s = run_big_s(params, vm_dev, K_dev, target_dev, max(5, args.steps // 2))
+                big_s = run_big_s(params, vm_dev, K_dev, target_dev, args.steps)
             except Exception as e:  # noqa: BLE001
                 big_s = {"error": f"{type(e).__name__}: {e}"[:300]}
             if not args.no_trainer:

@@ -15,7 +15,7 @@ by a 20-line shim restating its two published functions (render_weight_from_alph
 alpha * exclusive cumprod(1 - alpha) per ray; accumulate_along_rays = segment sum of
 weights * values) -- the reference's own alpha/sigma formula and autograd do the rest.
 
-Also writes tests/golden/garden.npz: the cropped assets/test_garden.npz scene
+Also writes tests/golden/garden_{0,1}.npz: the cropped assets/test_garden.npz scene
 (gsplat/_helper.py:51-102 load_test_data; crop [-2,2]^3 -> 111 785 points) so the GPU box,
 which has no /root/reference, can rebuild BASELINE.json's configs.  quats / scales /
 opacities are NOT stored: they are re-drawn with numpy's RandomState(42) by
@@ -94,15 +94,17 @@ def make_garden():
     d = np.load("/root/reference/assets/test_garden.npz")
     means = d["means3d"].astype(np.float32)
     sel = ((means >= -2.0) & (means <= 2.0)).all(-1)
+    h = int(sel.sum()) // 2  # two halves: every stored file stays below 1 MB (tests/scene.py joins them)
     save(
-        "garden.npz",
-        means=means[sel],
-        colors=d["colors"][sel],
+        "garden_0.npz",
+        means=means[sel][:h],
+        colors=d["colors"][sel][:h],
         viewmats=d["viewmats"].astype(np.float32),
         Ks=d["Ks"].astype(np.float32),
         width=np.int64(d["width"]),
         height=np.int64(d["height"]),
     )
+    save("garden_1.npz", means=means[sel][h:], colors=d["colors"][sel][h:])
     return means[sel], d["viewmats"].astype(np.float32), d["Ks"].astype(np.float32), int(d["width"]), int(d["height"])
 
 
@@ -369,7 +371,10 @@ def make_mcmc(rng):
 
 if __name__ == "__main__":
     if "--cameras-only" in sys.argv:  # adds the ortho / fisheye fixtures without rewriting the others
-        d = np.load(os.path.join(HERE, "garden.npz"))
+        sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+        from tests import scene
+
+        d = scene.load_garden()
         make_projection_cameras(d["means"], d["viewmats"], d["Ks"], int(d["width"]), int(d["height"]))
         sys.exit(0)
     rng = np.random.RandomState(20260922)

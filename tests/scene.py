@@ -1,7 +1,7 @@
 """Deterministic scene builder shared by tests, bench.py and __graft_entry__.smoke().
 
 Restates the recipe of the reference's ``load_test_data`` (/root/reference/gsplat/_helper.py:51-102):
-the [-2,2]^3 crop of assets/test_garden.npz (committed as tests/golden/garden.npz), optionally
+the [-2,2]^3 crop of assets/test_garden.npz (committed as tests/golden/garden_{0,1}.npz), optionally
 tiled ``scene_grid`` x ``scene_grid`` times, with random scales in [1e-4, 0.02], unit quaternions
 and opacities in [0,1).  Unlike the reference, the random attributes come from numpy's
 RandomState(seed) so that every machine (CPU container, GPU box) sees identical inputs.
@@ -18,8 +18,12 @@ SH_C0 = 0.28209479177387814
 
 
 def load_garden():
-    d = np.load(os.path.join(_GOLDEN, "garden.npz"))
-    return {k: d[k] for k in d.files}
+    """The crop is stored in two halves (garden_0.npz holds the cameras) to keep every stored file below 1 MB."""
+    parts = [np.load(os.path.join(_GOLDEN, f"garden_{i}.npz")) for i in range(2)]
+    g = {k: parts[0][k] for k in parts[0].files}
+    for k in ("means", "colors"):
+        g[k] = np.concatenate([p[k] for p in parts])
+    return g
 
 
 def make_scene(scene_grid: int = 1, n_max: int | None = None, sh_degree: int = 3, seed: int = 42):

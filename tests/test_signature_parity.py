@@ -1,12 +1,14 @@
 """Drop-in check of the operator surface: the public functions take exactly the reference's parameters, in the
-reference's order (parsed from the reference sources with `ast`; skipped where /root/reference is absent)."""
+reference's order.  The reference's side (nerfstudio-project/gsplat v1.6.0, parameter lists parsed from its sources
+with `ast`) is stored in tests/golden/ref_signatures.json."""
 import ast
+import json
 import os
 
 import pytest
 
-REF = "/root/reference/gsplat"
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+REF = json.load(open(os.path.join(ROOT, "tests", "golden", "ref_signatures.json")))
 
 
 def _params(path, fn):
@@ -18,7 +20,6 @@ def _params(path, fn):
     raise AssertionError(f"{fn} not found in {path}")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present")
 @pytest.mark.parametrize(
     "fn,ref_file,our_file",
     [
@@ -39,13 +40,14 @@ def _params(path, fn):
     ],
 )
 def test_same_parameters_as_reference(fn, ref_file, our_file):
-    ref, ref_defaults = _params(os.path.join(REF, ref_file), fn)
+    entry = REF["functions"][fn]
+    assert entry["file"] == "gsplat/" + ref_file
+    ref, ref_defaults = entry["params"], entry["n_defaults"]
     ours, our_defaults = _params(os.path.join(ROOT, "gsplat_b200", our_file), fn)
     assert ours == ref, f"{fn}: parameters differ\n reference: {ref}\n ours:      {ours}"
     assert our_defaults == ref_defaults, f"{fn}: number of defaulted parameters differs"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present")
 def test_rasterization_defaults_match_reference():
     def defaults(path):
         tree = ast.parse(open(path).read())
@@ -55,7 +57,7 @@ def test_rasterization_defaults_match_reference():
                 d = n.args.defaults
                 return {k: ast.unparse(v) for k, v in zip(names[len(names) - len(d):], d)}
 
-    ref = defaults(os.path.join(REF, "rendering.py"))
+    ref = REF["rasterization_defaults"]
     ours = defaults(os.path.join(ROOT, "gsplat_b200", "rendering.py"))
     # rolling_shutter: the reference's default is its RollingShutterType.GLOBAL enum member; ours is None (= global)
     diff = {k: (ref[k], ours.get(k)) for k in ref if ref[k] != ours.get(k) and k != "rolling_shutter"}
