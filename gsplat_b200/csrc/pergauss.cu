@@ -1829,20 +1829,10 @@ extern "C" int gsb200_isect_emit(
     const uint32_t tile_bits = bits_for_count((int64_t)tile_width * tile_height);
     if(bits_for_count(I) + tile_bits > 32)
         return GSB200_E_KEYBITS;
-    static const bool coop = [] {
-        const char *e = std::getenv("GSB200_EMIT");
-        return !(e && e[0] == 's'); // GSB200_EMIT=serial selects the one-thread-per-gaussian kernel (measurements)
-    }();
-    if(coop)
-        isect_emit_coop_kernel<int64_t><<<grid_for(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
-            total, N, means2d, radii, depths, conics, opacities, cum_tiles, image_ids, order, tile_size, tile_width, tile_height,
-            tile_bits, isect_ids, flatten_ids
-        );
-    else
-        isect_emit_kernel<int64_t><<<grid_for(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
-            total, N, means2d, radii, depths, conics, opacities, cum_tiles, image_ids, order, tile_size, tile_width, tile_height,
-            tile_bits, isect_ids, flatten_ids
-        );
+    isect_emit_coop_kernel<int64_t><<<grid_for(total, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+        total, N, means2d, radii, depths, conics, opacities, cum_tiles, image_ids, order, tile_size, tile_width, tile_height,
+        tile_bits, isect_ids, flatten_ids
+    );
     return check_launch();
 }
 

@@ -10,16 +10,18 @@
 //    contiguous float4 streams (cull: mean + conservative half extents of the alpha>=1/255 ellipse,
 //    geom: conic + opacity, color), so that every tile's list is a contiguous byte range;
 //  * each CTA (one 16x16 tile, 8 warps, a warp owns an 8x4 pixel block) streams its range through a
-//    2-stage shared-memory ring with 1-D TMA bulk copies (cp.async.bulk + mbarrier complete_tx);
+//    shared-memory ring filled with 1-D TMA bulk copies (cp.async.bulk + mbarrier complete_tx).  For
+//    D <= 4 channels the ring has 3 stages and no CTA barrier in the batch loop: every warp works at its
+//    own pace and the last warp out of a stage refills it.  For D > 4 the CTA moves through a 2-stage
+//    ring in step, with CTA barriers;
 //  * inside a batch every lane tests ONE gaussian's extent box against the warp's pixel block and the
 //    warp ballots: only gaussians that can reach alpha >= 1/255 inside the block are evaluated
 //    (exact: the skipped pairs are `continue`d by the reference too); finished warps drop out by ballot;
-//  * the backward walks the same ring back to front, reduces the 9(+2) per-gaussian partial sums of a
-//    warp with a butterfly transpose (12 shuffles instead of 45) and lets the lanes that end up owning
-//    a sum issue one red.global.add each.
+//  * the backward walks the same ring back to front with a transposed reduction: per surviving gaussian
+//    each lane (= pixel) buffers two scalars, and after 16 survivors each lane (= gaussian) sums its
+//    gaussian's gradient record over the warp's pixels and adds it with 128-bit red.global.add.
 #include <algorithm>
 
-#include <cstdlib>
 #include <mutex>
 
 #include "common.cuh"
@@ -522,257 +524,11 @@ __global__ void __launch_bounds__(kWarps * 32) raster_fwd_kernel(
 }
 
 // ---------------------------------------------------------------------------------------------
-// backward
-struct GradDst
-{
-    float *means2d, *conics, *colors, *opacities, *abs;
-    int64_t s_means2d, s_conics, s_colors, s_opacities, s_abs;
-};
-
-// MINB = CTAs per SM the register allocation is held to (48 registers at 5): the kernel is issue-bound, so
-// occupancy and code quality trade against each other; the host picks the variant (default 5 for CDIM <= 4,
-// GSB200_BWD_MINBLOCKS = 4 | 5 | 6 overrides it for measurements).
-template<int CDIM, bool ABS, int MINB>
-__global__ void __launch_bounds__(kWarps * 32, MINB) raster_bwd_kernel(
-    const uint32_t I, const int64_t n_isects, const float4 *__restrict__ gcull, const float4 *__restrict__ ggeom,
-    const float4 *__restrict__ gcolor, const int32_t *__restrict__ order, const int32_t *__restrict__ flatten_ids,
-    const float *__restrict__ backgrounds,
-    const uint8_t *__restrict__ masks, const uint32_t W, const uint32_t H, const uint32_t tw, const uint32_t th,
-    const int32_t *__restrict__ offsets, const float *__restrict__ render_alphas, const int32_t *__restrict__ last_ids,
-    const float *__restrict__ v_render_colors, const float *__restrict__ v_render_alphas, const GradDst dst
-)
-{
-    constexpr int CV = RecLayout<CDIM>::kColorVec4;
-    // slots: 0,1 = v_xy ; 2,3,4 = v_conic ; 5 = v_opacity ; 6..6+CDIM = v_rgb ; then 2 abs
-    constexpr int M = 6 + CDIM + (ABS ? 2 : 0);
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    Ring<CDIM> ring;
-    ring.carve(smem_raw);
-    __shared__ int32_t s_tile_bin;
-
-    const TileGeom tg      = decode_tile(order, tw, th);
-    const unsigned tid     = threadIdx.x;
-    const unsigned warp    = tid >> 5, lane = tid & 31;
-    const int64_t tile_lin = (int64_t)tg.image_id * tw * th + tg.tile_id;
-    if(masks != nullptr && !masks[tile_lin])
-        return;
-    const int32_t range_start = offsets[tile_lin];
-    const int32_t range_end0  = (tile_lin == (int64_t)I * tw * th - 1) ? (int32_t)n_isects : offsets[tile_lin + 1];
-    if(range_end0 <= range_start)
-        return;
-
-    const int bx0 = tg.tile_x * kTile + (warp & 1) * 8;
-    const int by0 = tg.tile_y * kTile + (warp >> 1) * 4;
-    const int px_i = bx0 + (lane & 7), py_i = by0 + (lane >> 3);
-    const float px = (float)px_i + 0.5f, py = (float)py_i + 0.5f;
-    const bool inside = (px_i < (int)W) && (py_i < (int)H);
-    const int64_t pix = inside ? ((int64_t)tg.image_id * H + py_i) * W + px_i : 0;
-    const float *bg   = backgrounds ? backgrounds + (size_t)tg.image_id * CDIM : nullptr;
-
-    const float T_final = inside ? 1.0f - render_alphas[pix] : 1.f;
-    float T             = T_final;
-    float buffer[CDIM], v_render_c[CDIM];
-    float bg_dot = 0.f;
-#pragma unroll
-    for(int k = 0; k < CDIM; ++k)
-    {
-        buffer[k]     = 0.f;
-        v_render_c[k] = inside ? v_render_colors[pix * CDIM + k] : 0.f;
-        if(bg)
-            bg_dot += bg[k] * v_render_c[k];
-    }
-    const float v_render_a       = (inside && v_render_alphas != nullptr) ? v_render_alphas[pix] : 0.f; // null: no gradient on alpha
-    const int32_t bin_final      = inside ? last_ids[pix] : -1;
-    const int32_t warp_bin_final = __reduce_max_sync(0xffffffffu, bin_final);
-
-    // nothing behind the tile's deepest contributor matters: shorten the list (block max of last_ids)
-    if(tid == 0)
-    {
-        s_tile_bin = -1;
-#pragma unroll
-        for(int s = 0; s < kStages; ++s)
-            mbar_init(ring.full(s), 1);
-        fence_mbar_init();
-    }
-    __syncthreads();
-    if(lane == 0)
-        atomicMax(&s_tile_bin, warp_bin_final);
-    __syncthreads();
-    const int32_t range_end = min(range_end0, s_tile_bin + 1);
-    if(range_end <= range_start)
-        return;
-
-    // which output(s) does this lane own after the butterfly reduction?  (two groups when M > 32)
-    constexpr int MA = M > 32 ? 32 : M;
-    constexpr int MB = M - MA;
-    auto slot_dst = [&](int slot, float *&p, int64_t &stride) {
-        p = nullptr, stride = 0;
-        if(slot < 0)
-            return;
-        if(slot < 2)
-            p = dst.means2d + slot, stride = dst.s_means2d;
-        else if(slot < 5)
-            p = dst.conics + (slot - 2), stride = dst.s_conics;
-        else if(slot == 5)
-            p = dst.opacities, stride = dst.s_opacities;
-        else if(slot < 6 + CDIM)
-            p = dst.colors + (slot - 6), stride = dst.s_colors;
-        else if(ABS)
-            p = dst.abs + (slot - 6 - CDIM), stride = dst.s_abs;
-    };
-    float *my_dst, *my_dst_b = nullptr;
-    int64_t my_stride64, my_stride_b64 = 0;
-    slot_dst(butterfly_slot<MA>(lane), my_dst, my_stride64);
-    if constexpr(MB > 0)
-    {
-        const int sb = butterfly_slot<MB>(lane);
-        slot_dst(sb >= 0 ? sb + MA : -1, my_dst_b, my_stride_b64);
-    }
-    // element offsets fit 32 bits (checked on the host: rows * stride < 2^32)
-    const uint32_t my_stride = (uint32_t)my_stride64, my_stride_b = (uint32_t)my_stride_b64;
-    uint32_t lane_r = lane, has_dst = my_dst != nullptr ? 1u : 0u;
-
-    const int num_batches = (range_end - range_start + kBatch - 1) / kBatch;
-    // batch b covers sorted indices [first, first + count), walking back to front
-    auto batch_first = [&](int b) -> int64_t {
-        const int64_t bf = (int64_t)range_end - (int64_t)(b + 1) * kBatch;
-        return bf > range_start ? bf : (int64_t)range_start;
-    };
-    auto batch_count = [&](int b) -> int {
-        return (int)((int64_t)range_end - (int64_t)b * kBatch - batch_first(b));
-    };
-
-    if(tid == 0)
-    {
-#pragma unroll
-        for(int s = 0; s < kStages; ++s)
-            if(s < num_batches)
-                ring.issue(s, gcull, ggeom, gcolor, batch_first(s), batch_count(s));
-    }
-    const float cx = (float)bx0 + 4.0f, cy = (float)by0 + 2.0f;
-
-    const float neg_Tf_bg = bg ? -T_final * bg_dot : 0.f;
-    const float Tf_va     = T_final * v_render_a + neg_Tf_bg; // T_final * (v_render_a - bg . v_render_c)
-    for(int b = 0; b < num_batches; ++b)
-    {
-        const int stage       = b % kStages;
-        const uint32_t parity = (uint32_t)(b / kStages) & 1u;
-        const int32_t first   = (int32_t)batch_first(b);
-        const int count       = batch_count(b);
-        // gaussian ids of this batch (coalesced; needed for the scatter)
-        if((int)tid < count)
-            ring.ids(stage)[tid] = flatten_ids[first + tid];
-        __syncthreads();
-        // the whole batch lies behind this warp's deepest contributor -> nothing to do for the warp
-        if(first <= warp_bin_final)
-        {
-            mbar_wait(ring.full(stage), parity);
-            const float4 *scull   = ring.cull(stage);
-            const float4 *saxis   = ring.axis(stage);
-            const float4 *sgeom   = ring.geom(stage);
-            const float4 *scol    = ring.color(stage);
-            const int32_t *sid    = ring.ids(stage);
-            int lim               = bin_final - first;      // local index of this pixel's last contributor
-            int warp_lim          = warp_bin_final - first; // ... of the warp's
-            // keep these loop invariants in registers: ptxas otherwise rematerialises them (64-bit batch arithmetic,
-            // S2R of the lane id, the ids pointer) once per surviving gaussian
-            uint32_t sid_addr = (uint32_t)__cvta_generic_to_shared(sid);
-            asm volatile("" : "+r"(lim), "+r"(warp_lim), "+r"(sid_addr), "+r"(lane_r), "+r"(has_dst));
-            for(int c1 = count; c1 > 0; c1 -= 32)
-            {
-                const int c0   = c1 - 32; // chunk covers local [c0, c1); c0 may be negative
-                const int mine = c0 + (int)lane;
-                bool hit       = false;
-                if(mine >= 0 && mine <= warp_lim)
-                    hit = block_may_touch(scull[mine], saxis[mine], cx, cy);
-                uint32_t mask = __ballot_sync(0xffffffffu, hit);
-                while(mask)
-                {
-                    const int j = 31 - __clz(mask); // back to front
-                    mask ^= 1u << j;
-                    const int t    = c0 + j;
-                    const float4 q = scull[t];
-                    const float4 g = sgeom[t];
-                    const float dx = q.x - px, dy = q.y - py;
-                    const float e2    = fmaf(g.x * dx, dx, fmaf(g.z * dy, dy, (g.y * dx) * dy)); // = -sigma * log2(e)
-                    const float vis   = fast_ex2(e2);
-                    const float ov    = g.w * vis;
-                    const float alpha = fminf(kMaxAlpha, ov);
-                    const bool valid  = (t <= lim) && e2 <= 0.f && alpha >= kAlphaThreshold;
-                    if(!__any_sync(0xffffffffu, valid))
-                        continue;
-                    float col[CV * 4];
-#pragma unroll
-                    for(int v = 0; v < CV; ++v)
-                    {
-                        const float4 cc = scol[t * CV + v];
-                        col[4 * v] = cc.x, col[4 * v + 1] = cc.y, col[4 * v + 2] = cc.z, col[4 * v + 3] = cc.w;
-                    }
-                    float part[M];
-#pragma unroll
-                    for(int k = 0; k < M; ++k)
-                        part[k] = 0.f;
-                    if(valid)
-                    {
-                        const float ra = fast_rcp(fmaxf(kMinOneMinusAlpha, 1.0f - alpha));
-                        T *= ra;
-                        const float fac = alpha * T;
-                        float v_alpha   = 0.f;
-#pragma unroll
-                        for(int k = 0; k < CDIM; ++k)
-                        {
-                            part[6 + k] = fac * v_render_c[k];
-                            v_alpha += (col[k] * T - buffer[k] * ra) * v_render_c[k];
-                            buffer[k] += col[k] * fac;
-                        }
-                        v_alpha += Tf_va * ra;
-                        if(ov <= kMaxAlpha)
-                        {
-                            const float v_sigma = -ov * v_alpha;
-                            const float ca = g.x * kConicUnscaleAC, cb = g.y * kConicUnscaleB, cc2 = g.z * kConicUnscaleAC;
-                            part[0]             = v_sigma * (ca * dx + cb * dy);
-                            part[1]             = v_sigma * (cb * dx + cc2 * dy);
-                            part[2]             = 0.5f * v_sigma * dx * dx;
-                            part[3]             = v_sigma * dx * dy;
-                            part[4]             = 0.5f * v_sigma * dy * dy;
-                            part[5]             = vis * v_alpha;
-                            if constexpr(ABS)
-                            {
-                                part[6 + CDIM]     = fabsf(part[0]);
-                                part[6 + CDIM + 1] = fabsf(part[1]);
-                            }
-                        }
-                    }
-                    Butterfly<MA, 16>::run(part, lane_r);
-                    uint32_t gid;
-                    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(gid) : "r"(sid_addr + 4u * (uint32_t)t));
-                    if(has_dst != 0u)
-                        atomicAdd(my_dst + (size_t)(gid * my_stride), part[0]);
-                    if constexpr(MB > 0)
-                    {
-                        Butterfly<MB, 16>::run(part + MA, lane);
-                        if(my_dst_b != nullptr)
-                            atomicAdd(my_dst_b + (size_t)(gid * my_stride_b), part[MA]);
-                    }
-                }
-            }
-        }
-        __syncthreads(); // stage (records + ids) fully consumed
-        if(tid == 0)
-        {
-            mbar_wait(ring.full(stage), parity); // landed even if every warp skipped it
-            if(b + kStages < num_batches)
-                ring.issue(stage, gcull, ggeom, gcolor, batch_first(b + kStages), batch_count(b + kStages));
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// backward, version 2: transposed reduction.
+// backward: transposed reduction.
 //
-// Version 1 above reduces the 9 (+2) per-pixel partials of every surviving (warp, gaussian) pair across the 32
-// lanes right away (butterfly: 12 shuffles + 12 adds + ~26 selects, 50 of its 130 instructions per survivor) and
-// issues 9 scalar REDs.  Version 2 splits the work in two phases per warp:
+// Reducing the 9 (+2) per-pixel partials of every surviving (warp, gaussian) pair across the 32 lanes right away
+// (butterfly: 12 shuffles + 12 adds + ~26 selects) costs 50 of 130 instructions per survivor, plus 9 scalar REDs.
+// Instead the work is split in two phases per warp:
 //   phase A (lane = pixel, sequential over the depth-sorted survivors, as before): per survivor each lane only
 //     computes TWO scalars -- f = alpha * T (the weight of the gaussian's colour in this pixel) and
 //     o = vis * v_alpha (gated like the reference gates v_sigma) -- and stores them into a per-warp shared
@@ -786,7 +542,13 @@ __global__ void __launch_bounds__(kWarps * 32, MINB) raster_bwd_kernel(
 //     compile-time immediates) and the D colour sums in registers -- no cross-lane traffic; the moments are
 //     re-centred on the gaussian's mean once per gaussian, the two halves are combined with one shuffle per
 //     value, and the 12-float gradient record is added with three 128-bit REDs instead of nine scalar ones.
-// Per survivor: ~45 + ~16 instructions instead of 130 (DESIGN.md section 3).
+// Per survivor: 52 + 18 instructions instead of 130 (SASS counts, DESIGN.md section 3).
+struct GradDst
+{
+    float *means2d, *conics, *colors, *opacities, *abs;
+    int64_t s_means2d, s_conics, s_colors, s_opacities, s_abs;
+};
+
 constexpr int kBwdBatch = 64; // records per ring stage (smaller than the forward's: the per-warp buffers need the room)
 constexpr int kRound    = 16; // survivors per reduction round of a warp
 constexpr int kRowF2    = 33; // row stride of the round buffer in float2 units (odd: conflict-free in both phases)
@@ -815,6 +577,7 @@ __device__ __forceinline__ void red_add_v4(float *addr, float a, float b, float 
 // the bulk copies of the batch three ahead.  Warps of a tile differ a lot in survivors per 64-record batch, and with
 // two CTA barriers per batch every warp ran at the pace of the slowest one.  The gaussian ids are read from global
 // memory when a survivor's data is materialised (no per-batch staging, hence no barrier for it either).
+// PIPE = false (D > 4): two CTA barriers per batch, the batch's gaussian ids staged in shared memory.
 template<int CDIM, bool ABS, int MINB, bool PIPE = false>
 __global__ void __launch_bounds__(kWarps * 32, MINB) raster_bwd2_kernel(
     const uint32_t I, const int64_t n_isects, const float4 *__restrict__ gcull, const float4 *__restrict__ ggeom,
@@ -1241,24 +1004,11 @@ static int launch_fwd(
         return rc;
     RecordStreams r      = carve_records(records, S, RecLayout<CDIM>::kColorVec4);
     const int32_t *order = (S > 0 && n_tiles >= 2 * 148) ? r.order : nullptr;
-    // default for CDIM <= 4: barrier-free ring (0.333 -> 0.304 ms incl. pack at cfg3); GSB200_FWD_PIPE=0 keeps the CTA barrier
-    static const bool pipe = [] {
-        const char *e = std::getenv("GSB200_FWD_PIPE");
-        return !(e && e[0] == '0');
-    }();
-    if(pipe && CDIM <= 4)
-    {
-        const size_t smem = ring_smem_bytes<CDIM, kBatch, kPipeStages>();
-        GSB_CUDA_TRY(cudaFuncSetAttribute(raster_fwd_kernel<CDIM, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        raster_fwd_kernel<CDIM, true><<<n_tiles, kWarps * 32, smem, st>>>(
-            (uint32_t)I, S, r.cull, r.geom, r.color, order, backgrounds, masks, W, H, tw, th, offsets, render_colors,
-            render_alphas, last_ids
-        );
-        return check_launch();
-    }
-    const size_t smem = ring_smem_bytes<CDIM>();
-    GSB_CUDA_TRY(cudaFuncSetAttribute(raster_fwd_kernel<CDIM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    raster_fwd_kernel<CDIM, false><<<n_tiles, kWarps * 32, smem, st>>>(
+    // CDIM <= 4: barrier-free ring (0.333 -> 0.304 ms incl. pack at cfg3 on a B200); CDIM > 4: the CTA-barrier ring
+    constexpr bool PIPE = CDIM <= 4;
+    const size_t smem   = ring_smem_bytes<CDIM, kBatch, PIPE ? kPipeStages : kStages>();
+    GSB_CUDA_TRY(cudaFuncSetAttribute(raster_fwd_kernel<CDIM, PIPE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    raster_fwd_kernel<CDIM, PIPE><<<n_tiles, kWarps * 32, smem, st>>>(
         (uint32_t)I, S, r.cull, r.geom, r.color, order, backgrounds, masks, W, H, tw, th, offsets, render_colors,
         render_alphas, last_ids
     );
@@ -1279,111 +1029,26 @@ static int launch_bwd(
     const unsigned n_tiles = (unsigned)(I * tw * th);
     const int32_t *order   = (n_tiles >= 2 * 148) ? r.order : nullptr; // written by the forward
     const bool absg        = dst.abs != nullptr;
-    // version 2 (transposed reduction) is the default; GSB200_BWD_ALGO=butterfly selects version 1 (measurements)
-    static const bool use_v2 = [] {
-        const char *e = std::getenv("GSB200_BWD_ALGO");
-        return !(e && e[0] == 'b');
-    }();
-    if(use_v2)
-    {
-        // are the five destinations one packed, 16-byte aligned record [v_xy 2 | v_conic 3 | v_opacity 1 | v_rgb D | abs 2]?
-        const int64_t P  = dst.s_means2d;
-        uint32_t packed  = 0;
-        if(P > 0 && (P % 4) == 0 && P >= 6 + CDIM + (absg ? 2 : 0) && dst.s_conics == P && dst.s_colors == P && dst.s_opacities == P
-           && dst.conics == dst.means2d + 2 && dst.opacities == dst.means2d + 5 && dst.colors == dst.means2d + 6
-           && (!absg || (dst.s_abs == P && dst.abs == dst.means2d + 6 + CDIM)) && (reinterpret_cast<uintptr_t>(dst.means2d) & 15) == 0)
-            packed = (uint32_t)P;
-        // GSB200_BWD_PIPE=0 keeps the two CTA barriers per batch (measurements); default: barrier-free ring
-        static const bool pipe = [] {
-            const char *e = std::getenv("GSB200_BWD_PIPE");
-            return !(e && e[0] == '0');
-        }();
-#define GSB_BWD2_LAUNCH(ABSV, MINBV, PIPEV)                                                                             \
-    do                                                                                                                  \
-    {                                                                                                                   \
-        const size_t smem2 = Bwd2Smem<CDIM, PIPEV>::total;                                                              \
-        GSB_CUDA_TRY(cudaFuncSetAttribute(                                                                              \
-            raster_bwd2_kernel<CDIM, ABSV, MINBV, PIPEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2       \
-        ));                                                                                                             \
-        raster_bwd2_kernel<CDIM, ABSV, MINBV, PIPEV><<<n_tiles, kWarps * 32, smem2, st>>>(                               \
-            (uint32_t)I, S, r.cull, r.geom, r.color, order, flatten_ids, backgrounds, masks, W, H, tw, th, offsets,     \
-            render_alphas, last_ids, v_render_colors, v_render_alphas, dst, packed                                      \
-        );                                                                                                              \
-    } while(0)
-        if constexpr(CDIM <= 4)
-        {
-            if(pipe)
-            {
-                if(absg)
-                    GSB_BWD2_LAUNCH(true, 4, true);
-                else
-                    GSB_BWD2_LAUNCH(false, 4, true);
-            }
-            else if(absg)
-                GSB_BWD2_LAUNCH(true, 4, false);
-            else
-                GSB_BWD2_LAUNCH(false, 4, false);
-        }
-        else
-        {
-            if(absg)
-                GSB_BWD2_LAUNCH(true, 1, false);
-            else
-                GSB_BWD2_LAUNCH(false, 1, false);
-        }
-#undef GSB_BWD2_LAUNCH
+    // are the five destinations one packed, 16-byte aligned record [v_xy 2 | v_conic 3 | v_opacity 1 | v_rgb D | abs 2]?
+    const int64_t P = dst.s_means2d;
+    uint32_t packed = 0;
+    if(P > 0 && (P % 4) == 0 && P >= 6 + CDIM + (absg ? 2 : 0) && dst.s_conics == P && dst.s_colors == P && dst.s_opacities == P
+       && dst.conics == dst.means2d + 2 && dst.opacities == dst.means2d + 5 && dst.colors == dst.means2d + 6
+       && (!absg || (dst.s_abs == P && dst.abs == dst.means2d + 6 + CDIM)) && (reinterpret_cast<uintptr_t>(dst.means2d) & 15) == 0)
+        packed = (uint32_t)P;
+    // CDIM <= 4: barrier-free ring, registers held to 4 CTAs / SM; CDIM > 4: the CTA-barrier ring
+    constexpr bool PIPE = CDIM <= 4;
+    constexpr int MINB  = CDIM <= 4 ? 4 : 1;
+    const size_t smem   = Bwd2Smem<CDIM, PIPE>::total;
+    auto launch = [&](auto kernel) -> int {
+        GSB_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kernel<<<n_tiles, kWarps * 32, smem, st>>>(
+            (uint32_t)I, S, r.cull, r.geom, r.color, order, flatten_ids, backgrounds, masks, W, H, tw, th, offsets,
+            render_alphas, last_ids, v_render_colors, v_render_alphas, dst, packed
+        );
         return check_launch();
-    }
-    const size_t smem  = ring_smem_bytes<CDIM>();
-#define GSB_BWD_LAUNCH(ABSV, MINBV)                                                                                     \
-    do                                                                                                                  \
-    {                                                                                                                   \
-        GSB_CUDA_TRY(cudaFuncSetAttribute(                                                                              \
-            raster_bwd_kernel<CDIM, ABSV, MINBV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem                \
-        ));                                                                                                             \
-        raster_bwd_kernel<CDIM, ABSV, MINBV><<<n_tiles, kWarps * 32, smem, st>>>(                                        \
-            (uint32_t)I, S, r.cull, r.geom, r.color, order, flatten_ids, backgrounds, masks, W, H, tw, th, offsets,     \
-            render_alphas, last_ids, v_render_colors, v_render_alphas, dst                                              \
-        );                                                                                                              \
-    } while(0)
-    if constexpr(CDIM <= 4)
-    {
-        static const int minb = [] {
-            const char *e = std::getenv("GSB200_BWD_MINBLOCKS");
-            const int v   = e ? std::atoi(e) : 5;
-            return (v == 4 || v == 6) ? v : 5;
-        }();
-        if(minb == 4)
-        {
-            if(absg)
-                GSB_BWD_LAUNCH(true, 4);
-            else
-                GSB_BWD_LAUNCH(false, 4);
-        }
-        else if(minb == 6)
-        {
-            if(absg)
-                GSB_BWD_LAUNCH(true, 6);
-            else
-                GSB_BWD_LAUNCH(false, 6);
-        }
-        else
-        {
-            if(absg)
-                GSB_BWD_LAUNCH(true, 5);
-            else
-                GSB_BWD_LAUNCH(false, 5);
-        }
-    }
-    else
-    {
-        if(absg)
-            GSB_BWD_LAUNCH(true, 1);
-        else
-            GSB_BWD_LAUNCH(false, 1);
-    }
-#undef GSB_BWD_LAUNCH
-    return check_launch();
+    };
+    return absg ? launch(raster_bwd2_kernel<CDIM, true, MINB, PIPE>) : launch(raster_bwd2_kernel<CDIM, false, MINB, PIPE>);
 }
 } // namespace gsb
 

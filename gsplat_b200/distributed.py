@@ -131,8 +131,8 @@ class NvlsGradArena:
     ALIGN = 64  # floats (256 B) between segment starts
 
     def __init__(
-        self, named_params: Dict[str, Tensor], group=None, blocks: Optional[int] = None, algo: Optional[str] = None,
-        row_sparse: Optional[bool] = None,
+        self, named_params: Dict[str, Tensor], group=None, blocks: int = 128, algo: Optional[str] = None,
+        row_sparse: bool = True,
     ):
         import torch.distributed._symmetric_memory as symm_mem
 
@@ -141,9 +141,7 @@ class NvlsGradArena:
         self.group = group if group is not None else dist.group.WORLD
         self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
         self.params = dict(named_params)
-        self.blocks = int(os.environ.get("GSB200_NVLS_BLOCKS", "128")) if blocks is None else int(blocks)
-        if row_sparse is None:
-            row_sparse = os.environ.get("GSB200_ALLREDUCE_ROWS", "1") != "0"
+        self.blocks = int(blocks)
         dev = next(iter(self.params.values())).device
         self.offsets, o = {}, 0
         for k, p in self.params.items():
@@ -166,7 +164,7 @@ class NvlsGradArena:
         self.flat = symm_mem.empty(self.numel, dtype=torch.float32, device=dev)
         self.hdl = symm_mem.rendezvous(self.flat, self.group.group_name)
         # world == 2: plain peer loads / stores move 1x the payload per direction, the multicast scheme 1.5x
-        self.algo = algo or os.environ.get("GSB200_ALLREDUCE_ALGO") or ("p2p" if self.world == 2 else "nvls")
+        self.algo = algo or ("p2p" if self.world == 2 else "nvls")
         if self.algo not in ("p2p", "nvls"):
             raise ValueError(f"unknown all-reduce algorithm {self.algo!r}")
         if self.algo == "nvls" and int(self.hdl.multicast_ptr) == 0:

@@ -829,10 +829,6 @@ def isect_tiles(
     return tiles_per_gauss, isect_ids, flatten_ids
 
 
-# GSB200_ISECT_SPECULATE=0: always read the totals before sizing the intersection stage (A/B runs)
-_SPECULATE = __import__("os").environ.get("GSB200_ISECT_SPECULATE", "1") != "0"
-
-
 class _IsectPredictor:
     """Capacities for gsb200_isect_sorted from the totals of the last calls on the same (device, image count, tile grid),
     and the asynchronous host read of the current totals (a kernel stores them into pinned memory, the host polls)."""
@@ -847,7 +843,7 @@ class _IsectPredictor:
         self.dev = dev
 
     def capacities(self, total_rows: int):
-        if not _SPECULATE or not self.hist:
+        if not self.hist:
             return None
         n_isects = max(h[0] for h in self.hist)
         n_vis = max(h[1] for h in self.hist)

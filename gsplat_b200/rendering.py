@@ -13,7 +13,6 @@ and raise NotImplementedError.
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, Optional, Tuple
 
 import torch
@@ -38,14 +37,6 @@ _HIT_DISTANCE_MODES = {"d", "Ed", "RGB-d", "RGB-Ed"}
 _DEPTH_MODES = {"D", "ED", "RGB+D", "RGB+ED"}
 _EXPECTED_MODES = {"Ed", "ED", "RGB-Ed", "RGB+ED"}
 _ALL_MODES = _COLOR_MODES | _HIT_DISTANCE_MODES | _DEPTH_MODES
-
-
-# GSB200_ISECT_WIDE=1 keeps the 64-bit (image | tile | depth) keys through the S-sized sort (round-1 pipeline; A/B runs)
-_ISECT_WIDE = os.environ.get("GSB200_ISECT_WIDE", "0") == "1"
-
-
-# GSB200_ROW_RECORDS=0: the fused projection neither counts tiles nor writes compositing row records (A/B runs)
-_NO_ROW_RECORDS = os.environ.get("GSB200_ROW_RECORDS", "1") == "0"
 
 
 class _Lazy:
@@ -330,7 +321,7 @@ def rasterization(
     else:
         # the fused projection can also count tiles and write the compositing row records, when what follows composites
         # exactly its outputs: plain RGB, input opacities (no antialiasing compensation), rows not exchanged between ranks
-        if render_mode == "RGB" and not antialiased and not sharded and not _ISECT_WIDE and not _NO_ROW_RECORDS:
+        if render_mode == "RGB" and not antialiased and not sharded:
             rows_out = RowSideOutputs(tile_size, math.ceil(width / float(tile_size)), math.ceil(height / float(tile_size)))
         radii, means2d, depths, conics, feat, compensations, opac = _project_dense(
             means, covars, quats, scales, opacities, colors, viewmats, Ks, width, height, sh_degree, eps2d, near_plane, far_plane,
@@ -384,11 +375,10 @@ def rasterization(
     tile_width = math.ceil(width / float(tile_size))
     tile_height = math.ceil(height / float(tile_size))
     # reference-shaped op sequence: (depth order,) count, emit, radix sort on the (image, tile) bits, offsets
-    if native_packed or _ISECT_WIDE:
+    if native_packed:
         tiles_per_gauss, isect_ids, flatten_ids = isect_tiles(
-            means2d, radii, depths, tile_size, tile_width, tile_height, sort=True, segmented=segmented, packed=native_packed,
-            n_images=I, image_ids=batch_ids * C + camera_ids if native_packed else None,
-            gaussian_ids=gaussian_ids if native_packed else None, conics=conics, opacities=opac,
+            means2d, radii, depths, tile_size, tile_width, tile_height, sort=True, segmented=segmented, packed=True,
+            n_images=I, image_ids=batch_ids * C + camera_ids, gaussian_ids=gaussian_ids, conics=conics, opacities=opac,
         )
         isect_offsets = isect_offset_encode(isect_ids, I, tile_width, tile_height)
     else:

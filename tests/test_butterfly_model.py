@@ -1,7 +1,8 @@
-"""CPU model of the butterfly ("transpose") warp reduction used by the backward rasterizer
-(gsplat_b200/csrc/common.cuh: Butterfly<M,16> + butterfly_slot<M>).  The recursion is restated in numpy
-with an explicit shfl_xor so that slot ownership and sums can be checked for every M the kernels use
-(M = 6 + channels [+ 2 for absgrad], and 12 for the pose gradient)."""
+"""CPU model of the butterfly ("transpose") warp reduction of the per-Gaussian backward
+(gsplat_b200/csrc/common.cuh: Butterfly<M,16> + butterfly_slot<M>; pergauss.cu uses M = 12 for the pose
+gradient and M = 3 for the view-direction sum).  The recursion is restated in numpy with an explicit
+shfl_xor so that slot ownership and sums can be checked; the template is generic in M, so a spread of
+M is checked, including M > 32."""
 import numpy as np
 import pytest
 
